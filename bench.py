@@ -2,6 +2,7 @@
 """Benchmark of the per-read simulation hot path (BASELINE.json metric: simulated bases/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload config2] [--batch_reads B]
+                    [--dump-outputs DIR]
 
 Workloads = the BASELINE.json configs, built by the SURVEY.md 8(d) generators (tests/synth.py):
 
@@ -283,6 +284,86 @@ class OraclePool:
             p.join(timeout=10)
 
 
+# --------------------------------------------------------------------------------------------------------------------
+# --dump-outputs: what the kernel-only arm left in a context's buffers after each batch of its last timed step
+# --------------------------------------------------------------------------------------------------------------------
+DUMP_READS = 1024       # reads sampled per batch (indices drawn with a fixed seed from the batch's read count)
+DUMP_BASES = 2048       # bases (and qualities) kept per sampled read: one window at a seeded position inside the read
+DUMP_LENGTHS = 1 << 20  # read lengths kept for the first DUMP_LENGTHS reads of a batch (all of them at the default sizes)
+READ_COLS = ["seq_len", "head", "tail", "n_pieces", "reversed", "flags", "attempts"]
+PIECE_COLS = ["read", "n_ops", "kind", "chrom", "pos", "ref_len", "out_len", "out_rel", "l_new", "ref_req", "ev_n_ops", "polya_len"]
+
+
+def device_bytes(ptr, n, dev):
+    """uint8 tensor over ``n`` bytes of device memory the library owns (no copy)."""
+    import torch
+
+    class View:
+        __cuda_array_interface__ = {"shape": (int(n),), "typestr": "|u1", "data": (int(ptr), False), "version": 3, "stream": None}
+    return torch.as_tensor(View(), device=dev)
+
+
+def snapshot_batch(eng, info, fastq, dev):
+    """Copies on the GPU, before the context runs its next batch, the batch's read and piece records and a window of
+    DUMP_BASES bases (and qualities) of DUMP_READS reads picked with a fixed seed.  Bounded work: a few MB."""
+    import torch
+    from nanosim_b200 import _lib as L
+
+    n, rb = int(info.n_reads), L.READ_DTYPE.itemsize
+    buf = eng.device_buffers()
+    reads = device_bytes(buf["reads"], n * rb, dev).clone()
+    pieces = device_bytes(buf["pieces"], int(info.n_pieces) * L.PIECE_DTYPE.itemsize, dev).clone()
+    rng = np.random.default_rng(0)
+    idx = np.sort(rng.choice(n, size=min(n, DUMP_READS), replace=False))
+    u = rng.random(len(idx))
+    ii = torch.from_numpy(idx).to(dev)
+    off = reads.view(torch.int64).view(n, rb // 8)[ii, 0]             # NsReadMeta: seq_off (u64), then seq_len (u32)
+    ln = reads.view(torch.int32).view(n, rb // 4)[ii, 2].long()
+    start = (torch.from_numpy(u).to(dev) * (ln - DUMP_BASES).clamp(min=0)).long()
+    col = torch.arange(DUMP_BASES, device=dev)
+    inside = col[None, :] < (ln - start)[:, None]
+    pos = torch.where(inside, (off + start)[:, None] + col[None, :], 0)
+    out = {"idx": idx, "start": start, "reads": reads, "pieces": pieces}
+    for key in ("seq", "qual") if fastq else ("seq",):
+        b = device_bytes(buf[key], int(info.seq_bytes), dev)
+        out[key] = torch.where(inside, b[pos], 0)
+    torch.cuda.current_stream(dev).synchronize()      # copies done before the context may overwrite its buffers
+    return out
+
+
+def write_dump(path, snaps, infos):
+    """DIR/<kind>_<name>.npy for the aligned and the unaligned batch of the last timed step (float32 / float64):
+    info (n_reads, n_pieces, total_bases, seq_bytes), read_len (the first DUMP_LENGTHS reads), sample (read indices),
+    reads and pieces (the sampled reads' records without buffer offsets, columns READ_COLS / PIECE_COLS; pieces[:, 0] is
+    the row of the read in `sample`), window_start, seq and qual (ASCII codes of each sampled read's window, 0 past the
+    read's end).  The edit scripts (ops) are deliberately left out: the bases, qualities and records they produce are
+    what a caller compares, and their layout may change between builds that emit the same reads."""
+    from nanosim_b200 import _lib as L
+
+    os.makedirs(path, exist_ok=True)
+    arrays = {}
+    for job, s in sorted(snaps.items()):
+        kind = "aligned" if job[0] == L.NS_KIND_ALIGNED else "unaligned"
+        info = infos[job]
+        reads = s["reads"].cpu().numpy().view(L.READ_DTYPE)
+        pieces = s["pieces"].cpu().numpy().view(L.PIECE_DTYPE)
+        sel = reads[s["idx"]]
+        rows = [(k, p) for k, r in enumerate(sel) for p in pieces[int(r["piece_first"]):int(r["piece_first"]) + int(r["n_pieces"])]]
+        arrays[kind + "_info"] = np.array([info.n_reads, info.n_pieces, info.total_bases, info.seq_bytes], dtype=np.float64)
+        arrays[kind + "_read_len"] = reads["seq_len"][:DUMP_LENGTHS].astype(np.float64)
+        arrays[kind + "_sample"] = s["idx"].astype(np.float64)
+        arrays[kind + "_reads"] = np.stack([sel[c].astype(np.float64) for c in READ_COLS], axis=1)
+        arrays[kind + "_pieces"] = np.array([[k] + [float(p[c]) for c in PIECE_COLS[1:]] for k, p in rows], dtype=np.float64).reshape(-1, len(PIECE_COLS))
+        arrays[kind + "_window_start"] = s["start"].cpu().numpy().astype(np.float64)
+        for key in ("seq", "qual"):
+            if key in s:
+                arrays[kind + "_" + key] = s[key].cpu().numpy().astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, "dump of %d bytes exceeds 64 MB" % total
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_sample_text(name, n_workers, per_worker, wall, worker_s, bases):
     extra = ""
     if WORKLOADS[name]["mode"] == "transcriptome":
@@ -308,7 +389,13 @@ def main():
     ap.add_argument("--cpu_reads", type=int, default=0, help="reads PER WORKER in a CPU-baseline step (0 = auto)")
     ap.add_argument("--cpu_procs", type=int, default=0, help="CPU-baseline worker processes (0 = all host cores)")
     ap.add_argument("--no_cpu_baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of what the kernel-only arm computed in its last step "
+                         "(rank 0) to DIR/<name>.npy, for comparing two builds output for output.  The sample is copied "
+                         "on the GPU inside the timed region, so the timing of a dump run is not one to compare")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -441,14 +528,30 @@ def main():
     if rank == 0:
         clocks.start()
     pipe.warm(jobs_for(range(1)))                   # every context sizes its buffers once (untimed)
-    pipe.run(jobs_for(range(args.warmup)), static_assign=static)
+    dump = bool(args.dump_outputs) and rank == 0
+    dump_jobs = set(jobs_for([args.warmup - 1])) if dump and args.warmup else set()
+    snaps, snap_infos = {}, {}
+
+    def keep_snapshot(e, info, job):
+        # a context's buffers are overwritten by its next batch: copy what the dump needs before the context moves on
+        if job in dump_jobs:
+            snaps[job], snap_infos[job] = snapshot_batch(e, info, W["fastq"], dev), info
+    # the last warm-up step is snapshotted too (and dropped), so that the copies' device memory is allocated before t0
+    pipe.run(jobs_for(range(args.warmup)), static_assign=static, after_simulate=keep_snapshot if dump else None)
+    if dump:
+        dump_jobs = set(jobs_for([total_steps - 1]))
+        snaps.clear()
+        snap_infos.clear()
     barrier()
     t0 = time.perf_counter()
-    rows = [row(i) for i in pipe.run(jobs_for(range(args.warmup, total_steps)), static_assign=static)]
+    rows = [row(i) for i in pipe.run(jobs_for(range(args.warmup, total_steps)), static_assign=static,
+                                     after_simulate=keep_snapshot if dump else None)]
     barrier()
     wall = time.perf_counter() - t0
     clocks.window(t0, t0 + wall, "kernel-only arm")
     pipe.close()
+    if dump:
+        write_dump(args.dump_outputs, snaps, snap_infos)
     if args.timeline and rank == 0:
         with open(args.timeline, "w") as f:       # phases are back to back on a context's stream: begin + cumulative durations
             f.write("reads\tbegin\tsetup_end\tplan_end\tscan_end\tscript_end\temit_end\n")

@@ -1,6 +1,7 @@
 """CPU tests of the host-side model compiler (nanosim_b200/model.py) against the oracle's own parsing/sampling."""
 import os
 import random
+import sys
 
 import numpy as np
 import pytest
@@ -122,10 +123,11 @@ def test_compiled_model_roundtrip(tmp_path, compiled_models):
         assert np.array_equal(cm.kde[k][0], cm2.kde[k][0]) and cm.kde[k][1] == cm2.kde[k][1]
 
 
-REF_MODELS = "/root/reference/pre-trained_models"
+# the original NanoSim's pre-trained_models/ directory (its model archives are hundreds of MB, not part of this repository)
+REF_MODELS = os.environ.get("NANOSIM_PRETRAINED_MODELS", "")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MODELS), reason="the reference's pre-trained models are only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF_MODELS), reason="set NANOSIM_PRETRAINED_MODELS to the original NanoSim's pre-trained_models directory")
 @pytest.mark.parametrize("tarball,prefix,shipped", [
     ("human_NA12878_DNA_FAB49712_guppy.tar.gz", "human_NA12878_DNA_FAB49712_guppy/training", "guppy_fab49712_plusq.npz"),
     ("human_NA12878_DNA_FAB49712_guppy_flipflop.tar.gz", "human_NA12878_DNA_FAB49712_guppy_flipflop/training", None),
@@ -147,3 +149,68 @@ def test_reference_model_directories_load_and_tabulate(tmp_path, tarball, prefix
             assert ours.text[k] == v, k
         for k, (data, bw) in cm.kde.items():
             assert np.array_equal(ours.kde[k][0], data) and ours.kde[k][1] == bw, k
+
+
+def _write_sklearn_kde_pickle(path, data, bandwidth, monkeypatch):
+    """joblib.dump of a KernelDensity as scikit-learn 0.22 lays it out: the estimator's __dict__ (bandwidth, kernel,
+    tree_, ...) with tree_ a KDTree reduced through ``newObj`` to the state tuple (data, idx_array, node_data,
+    node_bounds, leaf_size, ..., dist_metric).  Stand-in classes under the sklearn module names write the same globals
+    without scikit-learn installed."""
+    import joblib
+    import types
+
+    mods = {n: types.ModuleType(n) for n in ("sklearn", "sklearn.neighbors", "sklearn.neighbors._kde",
+                                             "sklearn.neighbors._kd_tree", "sklearn.neighbors._dist_metrics")}
+    for n, m in mods.items():
+        monkeypatch.setitem(sys.modules, n, m)
+
+    def newObj(cls):
+        return cls.__new__(cls)
+
+    class KDTree:
+        def __init__(self, state):
+            self.state = state
+
+        def __reduce__(self):
+            return newObj, (KDTree,), self.state
+
+    class EuclideanDistance:
+        def __reduce__(self):
+            return newObj, (EuclideanDistance,), {"p": 2.0}
+
+    class KernelDensity:
+        pass
+
+    for obj, mod in ((newObj, "_kd_tree"), (KDTree, "_kd_tree"), (EuclideanDistance, "_dist_metrics"), (KernelDensity, "_kde")):
+        obj.__module__, obj.__qualname__ = "sklearn.neighbors." + mod, obj.__name__
+        setattr(mods["sklearn.neighbors." + mod], obj.__name__, obj)
+    n = len(data)
+    kd = KernelDensity()
+    kd.__dict__.update(bandwidth=bandwidth, algorithm="auto", kernel="gaussian", metric="euclidean", atol=0, rtol=0,
+                       breadth_first=True, leaf_size=40, metric_params=None, _sklearn_version="0.22.1",
+                       tree_=KDTree((data, np.arange(n, dtype=np.intp), np.zeros(1), np.zeros((2, 1, data.shape[1])),
+                                     40, 1, 1, 0, 1, 0, 0, EuclideanDistance())))
+    joblib.dump(kd, path)
+
+
+@pytest.mark.parametrize("tag", CASES)
+def test_reference_format_directory_loads_as_shipped_model(tag, compiled_models, tmp_path, monkeypatch):
+    """`-c <dir>/<prefix>` with a model directory in the reference's on-disk format: text tables under their file names
+    and one KernelDensity pickle per KDE.  The directory is written from the shipped model, so load_model must return
+    it unchanged, and the device tables must build from it."""
+    from nanosim_b200.model import DeviceTables, load_model
+    cm = compiled_models[tag]
+    prefix = os.path.join(str(tmp_path), "training")
+    for name, text in cm.text.items():
+        with open(prefix + "_" + name, "w") as f:
+            f.write(text)
+    for name, (data, bw) in cm.kde.items():
+        _write_sklearn_kde_pickle(prefix + "_" + name + ".pkl", data, bw, monkeypatch)
+    monkeypatch.undo()                              # the stand-in modules are gone: the loader reads the pickles without them
+    got = load_model(prefix)
+    assert got.text == cm.text
+    assert sorted(got.kde) == sorted(cm.kde)
+    for k, (data, bw) in cm.kde.items():
+        assert got.kde[k][0].dtype == np.float64 and np.array_equal(got.kde[k][0], data) and got.kde[k][1] == bw, k
+    t = DeviceTables(got, fastq=True, chimeric="chimeric_info" in got.text)
+    assert len(t.alias_prob) > 1000 and len(got.kde) >= 5
